@@ -25,8 +25,10 @@ import argparse
 import hashlib
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -59,7 +61,14 @@ def parse_args():
                     help="N>1: strong = the same read set split over the ranks (default); weak = every rank brings its own --genome/N ... see --weak-genome")
     ap.add_argument("--weak-genome", type=int, default=0, help="weak scaling / configs[2]: TOTAL genome size; every rank generates and feeds 1/N of the reads")
     ap.add_argument("--write-digest", action="store_true", help="record this run's distinct count + histogram hash as the golden digest of the workload")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64): coverage_hist "
+                         "(256 counts of distinct k-mers by coverage, 255 = saturated) and pass1_counts (records, reads kept, k-mer "
+                         "instances, distinct k-mers, linear nodes marked, k-mers removed)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------- synthetic reads (torch = plumbing)
@@ -259,8 +268,18 @@ def main():
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
-    workdir = os.environ.get("PGB200_BENCH_DIR", "/tmp/pgb200_bench")
+    # scratch for the reference arm's read files: a private temporary directory unless PGB200_BENCH_DIR names one
+    own_workdir = "PGB200_BENCH_DIR" not in os.environ
+    workdir = tempfile.mkdtemp(prefix="pgb200_bench_") if own_workdir else os.environ["PGB200_BENCH_DIR"]
     os.makedirs(workdir, exist_ok=True)
+    try:
+        run(args, torch, workdir, rank, world, local_rank)
+    finally:
+        if own_workdir:
+            shutil.rmtree(workdir, ignore_errors=True)
+
+
+def run(args, torch, workdir, rank, world, local_rank):
     weak = args.scale == "weak" or args.weak_genome > 0
     total_genome = args.weak_genome if args.weak_genome > 0 else (args.genome * world if weak else args.genome)
     workload = f"synthetic {total_genome/1e6:g} Mbp genome, {args.coverage:g}x {RD_LEN} bp PE FASTQ (insert {INSERT}, {ERR*100:g}% subst.), K={K}"
@@ -369,11 +388,11 @@ def main():
         if timeline is not None:
             for j in range(5):
                 timeline[j] += tl[j + 1] - tl[j]
-        return st, hist
+        return st, hist, lin, rem
 
     def timed(bufs, on_device, steps, warmup):
         for _ in range(warmup):
-            st, hist = one_step(bufs, on_device)
+            one_step(bufs, on_device)
         if timeline is not None:
             for j in range(5):
                 timeline[j] = 0.0
@@ -384,7 +403,7 @@ def main():
         e0.record()
         t0 = time.perf_counter()
         for _ in range(steps):
-            st, hist = one_step(bufs, on_device)
+            st, hist, lin, rem = one_step(bufs, on_device)
             ins_ms += st.ms_insert
             app_ms += st.ms_apply
             dec_ms += st.ms_decode
@@ -405,10 +424,13 @@ def main():
             sm = tt.clone(); dist.all_reduce(sm, op=dist.ReduceOp.SUM)
             ms, distinct, instances, ins_ms, app_ms, dec_ms = mx[0].item(), sm[1].item(), sm[2].item(), mx[3].item(), mx[4].item(), mx[5].item()
             hh = torch.tensor(hist, device=dev, dtype=torch.int64); dist.all_reduce(hh); hist = hh.tolist()
+            cc = torch.tensor([st.records, st.reads_kept, lin, rem], device=dev, dtype=torch.int64); dist.all_reduce(cc)
+            records, reads_kept, lin, rem = cc.tolist()
         else:
-            distinct, instances = st.distinct, st.instances
+            distinct, instances, records, reads_kept = st.distinct, st.instances, st.records, st.reads_kept
+        counts = [records, reads_kept, int(instances), int(distinct), lin, rem]   # the job's, as --dump-outputs writes them
         return {"ms": ms / steps, "distinct": int(distinct), "instances": int(instances), "ins_ms": ins_ms / steps, "app_ms": app_ms / steps,
-                "dec_ms": dec_ms / steps, "launches": launches // steps, "hist": hist, "st": st}
+                "dec_ms": dec_ms / steps, "launches": launches // steps, "hist": hist, "counts": counts, "st": st}
 
     with ClockSampler(local_rank) as cs:
         r = timed((t1, t2), True, args.steps, args.warmup)
@@ -433,6 +455,11 @@ def main():
         json.dump(known, open(DIGESTS, "w"), indent=1, sort_keys=True)
     assert r["instances"] == total_instances, (r["instances"], total_instances)
     assert sum(r["hist"]) == r["distinct"]
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "coverage_hist.npy"), np.asarray(r["hist"], dtype=np.float64))
+        np.save(os.path.join(args.dump_outputs, "pass1_counts.npy"), np.asarray(r["counts"], dtype=np.float64))
 
     e2e = None
     if not args.no_e2e:

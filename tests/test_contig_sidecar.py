@@ -20,10 +20,15 @@ OUT = ["contig", "Arc", "updated.edge", "ContigIndex"]
 
 
 @pytest.fixture(scope="module", autouse=True)
-def _need():
+def _build():
     subprocess.run(["make", "-s", "-j8", "-C", os.path.join(util.ROOT, "soapdenovo2_b200", "csrc")], check=True)
+
+
+@pytest.fixture(scope="module")
+def _dropin():
+    """The drop-in binaries are linked from the reference's own objects: only where oracle/Makefile could build those."""
     if not (util.have_ref() and os.path.isdir(os.path.join(util.ROOT, "oracle", "_ref", "o63"))):
-        pytest.skip("oracle/_ref absent (built where /root/reference exists)")
+        pytest.skip("oracle/_ref absent (the reference's objects are built by `make -C oracle ref` where its sources are)")
     subprocess.run(["bash", os.path.join(util.ROOT, "scripts", "link_dropin.sh")], check=True, capture_output=True)
 
 
@@ -34,7 +39,7 @@ def _copy_pregraph(src, dst):
 
 
 @pytest.mark.parametrize("flav,K,extra", [(0, 63, ("-R",)), (0, 31, ()), (1, 91, ("-R",))])
-def test_contig_reads_the_sidecar(tmp_path, flav, K, extra):
+def test_contig_reads_the_sidecar(_dropin, tmp_path, flav, K, extra):
     cfg = synth.scenario_multilib(str(tmp_path)) if K != 31 else synth.scenario_se_fasta(str(tmp_path))
     ref_bin, b200_bin = (util.REF127, B127) if flav else (util.REF63, B63)
     ref = str(tmp_path / "ref")

@@ -8,24 +8,19 @@ import pytest
 
 from soapdenovo2_b200 import api, synth
 from tests import util
-from tests.test_gpu_full import _engine, _oracle
+from tests.test_gpu_full import _engine, _oracle, _suffixes
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module", autouse=True)
-def _build():
-    util.build_oracle()
 
 
 @pytest.mark.parametrize("crlf,K,P,extra", [(False, 31, 3, ("-R",)), (True, 31, 8, ("-a", "1", "-d", "2")), (True, 63, 4, ("-a", "1", "-R")),
                                             (False, 13, 2, ("-a", "1", "-R"))])
 def test_adversarial_inputs(tmp_path, crlf, K, P, extra):
     cfg = synth.scenario_adversarial(str(tmp_path), crlf=crlf, K_hint=max(K, 31))
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(0, cfg, ref, K, P, extra)
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle(util.adversarial_name(crlf, max(K, 31)), cfg, 0, K, P, extra)
     _engine(0, cfg, gpu, K, P, extra)
-    util.compare(ref, gpu, util.SUFFIXES_R if "-R" in extra else util.SUFFIXES)
+    util.compare_golden(gpu, rec, _suffixes(extra))
 
 
 def test_saturation_under_contention():

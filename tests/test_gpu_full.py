@@ -1,5 +1,6 @@
-"""GPU parity, whole stage: `pregraph-b200-{63,127}mer pregraph ...` must write the same bytes as the reference binary
-(oracle/_ref, shipped prebuilt) -- or as the C model where the reference was not shipped -- for all seven files."""
+"""GPU parity, whole stage: `pregraph-b200-{63,127}mer pregraph ...` must write the same bytes as the reference binary for all
+seven files, and print the same counters.  The reference's outputs are the SHA-256 digests and counter lines stored in
+tests/golden/reference_outputs.json (scripts/make_reference_golden.py)."""
 import os
 import subprocess
 
@@ -11,15 +12,13 @@ from tests import util
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(scope="module", autouse=True)
-def _build():
-    util.build_oracle()
+def _oracle(scenario, cfg, flavour127, K, P, extra):
+    """The reference's record for this run (output digests, counter lines)."""
+    return util.golden(scenario, flavour127, K, P, extra, cfg=cfg)
 
 
-def _oracle(flavour127, cfg, out, K, P, extra):
-    if util.have_ref():
-        return util.run_ref(util.REF127 if flavour127 else util.REF63, cfg, out, K, P, extra)
-    return util.run_model(util.MODEL127 if flavour127 else util.MODEL63, cfg, out, K, P, extra)
+def _suffixes(extra):
+    return util.SUFFIXES_R if "-R" in extra else util.SUFFIXES
 
 
 def _engine(flavour127, cfg, out, K, P, extra, env=None):
@@ -28,11 +27,6 @@ def _engine(flavour127, cfg, out, K, P, extra, env=None):
                        env=dict(os.environ, **(env or {})), timeout=900)
     assert r.returncode == 0, r.stderr[-4000:]
     return r.stderr
-
-
-def _counter_lines(log):
-    keep = ("node(s) allocated", "tip(s) removed", "linear node(s) marked", "edge(s) and", "vertex(es) output", "pre-arc(s) added", "kmer(s) removed")
-    return [l.strip() for l in log.splitlines() if any(k in l for k in keep)]
 
 
 @pytest.fixture(scope="module")
@@ -47,94 +41,86 @@ def pe_cfg(tmp_path_factory):
 
 @pytest.mark.parametrize("K,P,extra", [(31, 3, ("-a", "1", "-R")), (31, 8, ("-a", "1", "-d", "1", "-R")), (31, 1, ("-a", "1")), (21, 5, ("-a", "1", "-d", "3"))])
 def test_se_fasta(se_cfg, tmp_path, K, P, extra):
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    lr = _oracle(0, se_cfg, ref, K, P, extra)
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("se", se_cfg, 0, K, P, extra)
     lg = _engine(0, se_cfg, gpu, K, P, extra)
-    util.compare(ref, gpu, util.SUFFIXES_R if "-R" in extra else util.SUFFIXES)
-    if util.have_ref():
-        assert _counter_lines(lr) == _counter_lines(lg)
+    util.compare_golden(gpu, rec, _suffixes(extra))
+    assert rec["counters"] == util.counter_lines(lg)
 
 
 @pytest.mark.parametrize("P,extra", [(8, ("-a", "1", "-R")), (4, ("-a", "1"))])
 def test_pe_fastq_k63(pe_cfg, tmp_path, P, extra):
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(0, pe_cfg, ref, 63, P, extra)
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("pe", pe_cfg, 0, 63, P, extra)
     _engine(0, pe_cfg, gpu, 63, P, extra)
-    util.compare(ref, gpu, util.SUFFIXES_R if "-R" in extra else util.SUFFIXES)
+    util.compare_golden(gpu, rec, _suffixes(extra))
 
 
 @pytest.mark.parametrize("K,P,extra", [(127, 3, ("-a", "1", "-R")), (91, 8, ("-a", "1")), (63, 2, ("-a", "1", "-R"))])
 def test_127mer_flavour(pe_cfg, tmp_path, K, P, extra):
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(1, pe_cfg, ref, K, P, extra)
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("pe", pe_cfg, 1, K, P, extra)
     _engine(1, pe_cfg, gpu, K, P, extra)
-    util.compare(ref, gpu, util.SUFFIXES_R if "-R" in extra else util.SUFFIXES)
+    util.compare_golden(gpu, rec, _suffixes(extra))
 
 
 def test_multilib_k63_small_chunks(tmp_path):
     """4 libraries (FASTA/FASTQ, SE/PE, rd_len_cutoff, reverse_seq, N's, lower case, ignored asm_flags=2 lib); 1 MB host chunks."""
     cfg = synth.scenario_multilib(str(tmp_path))
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(0, cfg, ref, 63, 8, ("-a", "1", "-R"))
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("multilib", cfg, 0, 63, 8, ("-a", "1", "-R"))
     _engine(0, cfg, gpu, 63, 8, ("-a", "1", "-R"), env={"PGB200_CHUNK_MB": "1", "PGB200_TABLE_SLOTS": "4096"})
-    util.compare(ref, gpu, util.SUFFIXES_R)
+    util.compare_golden(gpu, rec, util.SUFFIXES_R)
 
 
 def test_multilib_k63_aggregated_pass1(tmp_path):
     """The same multi-library case with pass 1 forced through the aggregated path (super-k-mer records, skm.cu), several chunks."""
     cfg = synth.scenario_multilib(str(tmp_path))
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(0, cfg, ref, 63, 8, ("-a", "1", "-R"))
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("multilib", cfg, 0, 63, 8, ("-a", "1", "-R"))
     _engine(0, cfg, gpu, 63, 8, ("-a", "1", "-R"), env={"PGB200_SKM": "1", "PGB200_CHUNK_MB": "1", "PGB200_TABLE_SLOTS": "4096"})
-    util.compare(ref, gpu, util.SUFFIXES_R)
+    util.compare_golden(gpu, rec, util.SUFFIXES_R)
 
 
 def test_downstream_contig_consumes_gpu_output(tmp_path):
-    """configs[4]: the reference's own `contig` stage must produce identical contigs from both pregraph outputs."""
-    if not util.have_ref():
-        pytest.skip("oracle/_ref not shipped")
+    """configs[4]: the reference's own `contig` stage must produce identical contigs from both pregraph outputs.  The contig
+    stage is a deterministic function of the pregraph files, so byte identity with the reference's pregraph files carries over to
+    the contigs the golden record holds; where the reference binary is built, its `contig` runs on the GPU output as well."""
     cfg = synth.scenario_multilib(str(tmp_path))
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    util.run_ref(util.REF63, cfg, ref, 63, 8, ("-a", "1", "-R"))
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("multilib", cfg, 0, 63, 8, ("-a", "1", "-R"))
     _engine(0, cfg, gpu, 63, 8, ("-a", "1", "-R"))
-    for pre in (ref, gpu):
-        util.run([util.REF63, "contig", "-g", pre, "-R"])
-    util.compare(ref, gpu, ["contig", "Arc", "updated.edge", "ContigIndex"])
+    util.compare_golden(gpu, rec, util.SUFFIXES_R)
+    if util.have_ref():
+        util.run([util.REF63, "contig", "-g", gpu, "-R"])
+        util.compare_golden(gpu, rec, util.CONTIG_SUFFIXES)
 
 
 def test_midsize_pe_k63_vs_reference(tmp_path):
     """2 Mbp genome, 30x, 150 bp PE FASTQ, K=63, -p 8 -a 2 -R (17.6 M k-mer instances): exercises many tip rounds, long edges."""
-    import numpy as np
-    g = synth.genome(2_000_000, 11, repeat=(2000, 4))
-    r1, r2 = synth.pe_reads(g, 200_000, 150, 300, 0.001, 12)
-    d = str(tmp_path)
-    synth.write_fastq(os.path.join(d, "a_1.fq"), r1, "m")
-    synth.write_fastq(os.path.join(d, "a_2.fq"), r2, "m")
-    cfg = os.path.join(d, "mid.cfg")
-    synth.write_config(cfg, 150, [{"avg_ins": 300, "files": [("q1", os.path.join(d, "a_1.fq")), ("q2", os.path.join(d, "a_2.fq"))]}])
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    lr = _oracle(0, cfg, ref, 63, 8, ("-a", "2", "-R"))
+    cfg = util.scenario_midsize(str(tmp_path))
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("mid", cfg, 0, 63, 8, ("-a", "2", "-R"))
     lg = _engine(0, cfg, gpu, 63, 8, ("-a", "2", "-R"))
-    util.compare(ref, gpu, util.SUFFIXES_R)
-    if util.have_ref():
-        assert _counter_lines(lr) == _counter_lines(lg)
+    util.compare_golden(gpu, rec, util.SUFFIXES_R)
+    assert rec["counters"] == util.counter_lines(lg)
     # and with the aggregated pass 1 (forced: the CLI feeds host text, which defaults to per-chunk inserts)
     gpu2 = str(tmp_path / "gpu2")
     _engine(0, cfg, gpu2, 63, 8, ("-a", "2", "-R"), env={"PGB200_SKM": "1"})
-    util.compare(ref, gpu2, util.SUFFIXES_R)
+    util.compare_golden(gpu2, rec, util.SUFFIXES_R)
 
 
 @pytest.mark.parametrize("K,P,extra", [(31, 3, ("-R",)), (31, 8, ()), (31, 1, ("-d", "1"))])
 def test_dynamic_tables_no_a(se_cfg, tmp_path, K, P, extra):
     """f1: without -a the reference's sets grow (in-place rehash with displacement chains); the engine replays the growth history."""
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(0, se_cfg, ref, K, P, extra)
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("se", se_cfg, 0, K, P, extra)
     _engine(0, se_cfg, gpu, K, P, extra)
-    util.compare(ref, gpu, util.SUFFIXES_R if "-R" in extra else util.SUFFIXES)
+    util.compare_golden(gpu, rec, _suffixes(extra))
 
 
 def test_dynamic_tables_no_a_pe_127(pe_cfg, tmp_path):
-    ref, gpu = str(tmp_path / "ref"), str(tmp_path / "gpu")
-    _oracle(1, pe_cfg, ref, 127, 4, ("-R",))
+    gpu = str(tmp_path / "gpu")
+    rec = _oracle("pe", pe_cfg, 1, 127, 4, ("-R",))
     _engine(1, pe_cfg, gpu, 127, 4, ("-R",))
-    util.compare(ref, gpu, util.SUFFIXES_R)
+    util.compare_golden(gpu, rec, util.SUFFIXES_R)

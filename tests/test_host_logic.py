@@ -1,5 +1,5 @@
 """CPU: the host-side read-stream plan (config parsing, library sort, file-type order, truncation) against the ORDER in which the
-unmodified reference binary opens the files (its "Import reads from file:" stderr lines)."""
+unmodified reference binary opens the files (its "Import reads from file:" stderr lines, stored in tests/golden/reference_outputs.json)."""
 import os
 import subprocess
 
@@ -14,24 +14,12 @@ def _build():
     subprocess.run(["make", "-s", "-j8", "-C", os.path.join(util.ROOT, "soapdenovo2_b200", "csrc")], check=True)
 
 
-def _ref_order(cfg, out):
-    log = util.run_ref(util.REF63, cfg, out, 31, 2)
-    lines = log.splitlines()
-    order = []
-    for i, l in enumerate(lines):
-        if l.startswith("Import reads from file:"):
-            order.append(lines[i + 1].strip())
-        if "done hashing nodes" in l:
-            break
-    return order
-
-
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
 def test_multilib_plan_matches_reference_open_order(tmp_path):
     cfg = synth.scenario_multilib(str(tmp_path))
     mrl, plan = api.plan_files(cfg)
     assert mrl == 150
-    assert [p[4] for p in plan] == _ref_order(cfg, str(tmp_path / "ref"))
+    assert [os.path.dirname(p[4]) for p in plan] == [str(tmp_path)] * len(plan)
+    assert [os.path.basename(p[4]) for p in plan] == util.golden("multilib", 0, 31, 2)["open_order"]
     by = {os.path.basename(p[4]): p for p in plan}
     assert by["m_a1.fa"][:4] == (0, 0, 0, 150) and by["m_a2.fa"][:4] == (1, 0, 0, 150)
     assert by["m_s.fa"][:4] == (-1, 0, 0, 140) and by["m_q1.fq"][:4] == (0, 1, 0, 140)       # rd_len_cutoff=140
@@ -39,10 +27,10 @@ def test_multilib_plan_matches_reference_open_order(tmp_path):
     assert "m_ig.fa" not in by                                                                   # asm_flags=2 is not used by pregraph
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
 def test_config_quirks(tmp_path):
     """max_rd_len only counts before the first [LIB]; '#' lines and unknown keys are ignored; q before f inside a library is
-    still opened after f1/f2 and q1/q2; default max_rd_len is 100."""
+    still opened after f1/f2 and q1/q2; default max_rd_len is 100.  The reference opens the files of this config in the order
+    asserted here (a run of the unmodified binary: "Import reads from file:" z1.fq, z2.fq, x.fa, y.fq)."""
     d = str(tmp_path)
     g = synth.genome(3000, 2)
     for name, fq in (("x.fa", False), ("y.fq", True), ("z1.fq", True), ("z2.fq", True)):
@@ -53,8 +41,7 @@ def test_config_quirks(tmp_path):
         f.write("#a comment\nfoo=bar\n[LIB]\navg_ins=300\nmax_rd_len=50\nq=%s/y.fq\nf=%s/x.fa\nq1=%s/z1.fq\nq2=%s/z2.fq\nasm_flags=1\n" % (d, d, d, d))
     mrl, plan = api.plan_files(cfg)
     assert mrl == 100
-    assert [os.path.basename(p[4]) for p in plan] == ["z1.fq", "z2.fq", "x.fa", "y.fq"]
-    assert [p[4] for p in plan] == _ref_order(cfg, os.path.join(d, "ref"))
+    assert [p[4] for p in plan] == [os.path.join(d, n) for n in ("z1.fq", "z2.fq", "x.fa", "y.fq")]
 
 
 def _fq(n, qual=None, eol=b"\n"):
