@@ -1,12 +1,14 @@
 #!/usr/bin/env python
-"""Fuzz the CPU oracle (oracle/pregraph_model.c) against the unmodified reference binary on random small scenarios: random genome /
-read geometry / error rate, K, -p, -a, -d, -R, 63- and 127-mer builds.  CPU only; `python scripts/fuzz_oracle.py [n_cases] [seed0]`.
+"""Fuzz the CPU oracle (oracle/pregraph_model.c) against the unmodified reference binary on the seeded random scenarios of
+synth.scenario_fuzz: read formats, libraries, ragged / long / truncated reads, CRLF, unusual bytes, K, -p, -a, -d, -R, 63- and
+127-mer builds.  CPU only; `python scripts/fuzz_oracle.py [n_cases] [seed0] [-j jobs]`.
 Prints one line per case and the mismatching suffixes, exit code 1 if any case differs."""
+import argparse
+import filecmp
 import os
 import sys
 import tempfile
-
-import numpy as np
+from concurrent.futures import ThreadPoolExecutor
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -15,53 +17,34 @@ from tests import util               # noqa: E402
 
 
 def one_case(seed: int):
-    rng = np.random.default_rng(seed)
-    kind = int(rng.integers(0, 4))
-    big = bool(rng.integers(0, 2))
-    K = int(rng.choice([13, 15, 21, 23, 31, 33, 45, 61, 63] if not big else [65, 77, 91, 99, 125, 127]))
-    P = int(rng.choice([1, 2, 3, 4, 5, 8, 16]))
-    extra = []
-    if rng.random() < 0.6:
-        extra += ["-a", str(int(rng.choice([1, 2])))]
-    if rng.random() < 0.4:
-        extra += ["-d", str(int(rng.integers(1, 4)))]
-    if rng.random() < 0.6:
-        extra += ["-R"]
     with tempfile.TemporaryDirectory() as d:
-        if kind == 0:
-            rd = int(rng.choice([K + 1, K + 5, 100, 150])) if K < 100 else int(rng.choice([K + 1, 150]))
-            cfg = synth.scenario_se_fasta(d, genome_len=int(rng.integers(3000, 30000)), n_reads=int(rng.integers(200, 4000)), rd_len=max(rd, K + 1),
-                                          err=float(rng.choice([0.0, 0.002, 0.01])), seed=seed)
-        elif kind == 1:
-            rd = int(rng.choice([100, 125, 150])) if K < 100 else 150
-            cfg = synth.scenario_pe_fastq(d, genome_len=int(rng.integers(5000, 60000)), n_pairs=int(rng.integers(300, 5000)), rd_len=rd,
-                                          insert=int(rng.integers(rd + 10, 500)), err=float(rng.choice([0.0, 0.003, 0.008])), seed=seed,
-                                          repeat=(int(rng.integers(100, 600)), int(rng.integers(1, 4))))
-        elif kind == 2:
-            cfg = synth.scenario_multilib(d, genome_len=int(rng.integers(10000, 50000)), seed=seed)
-        else:
-            K = min(K, 99)   # its reads are at most 100 bases long (the reference itself fails on a library without a single k-mer)
-            cfg = synth.scenario_adversarial(d, seed=seed, crlf=bool(rng.integers(0, 2)), K_hint=min(K, 97))
+        cfg, K, big, P, extra, _env = synth.scenario_fuzz(d, seed)
         ref_bin, mod_bin = (util.REF127, util.MODEL127) if big else (util.REF63, util.MODEL63)
         ref, mod = os.path.join(d, "ref"), os.path.join(d, "mod")
-        util.run_ref(ref_bin, cfg, ref, K, P, tuple(extra))
-        util.run_model(mod_bin, cfg, mod, K, P, tuple(extra))
+        util.run_ref(ref_bin, cfg, ref, K, P, extra)
+        util.run_model(mod_bin, cfg, mod, K, P, extra)
         sfx = util.SUFFIXES_R if "-R" in extra else util.SUFFIXES
-        import filecmp
         bad = [s for s in sfx if not filecmp.cmp(f"{ref}.{s}", f"{mod}.{s}", shallow=False)]
-    return f"seed {seed} kind {kind} K {K} P {P} {' '.join(extra)}", bad
+    return f"seed {seed} {'127' if big else '63'}mer K {K} P {P} {' '.join(extra)}", bad
+
+
+def checked(seed: int):
+    try:
+        return one_case(seed)
+    except Exception as e:   # a crash of either binary is a finding too
+        return f"seed {seed}", [f"EXCEPTION {str(e)[-300:]}"]
 
 
 if __name__ == "__main__":
-    n = int(sys.argv[1]) if len(sys.argv) > 1 else 40
-    s0 = int(sys.argv[2]) if len(sys.argv) > 2 else 1000
+    ap = argparse.ArgumentParser()
+    ap.add_argument("n", type=int, nargs="?", default=40)
+    ap.add_argument("seed0", type=int, nargs="?", default=1000)
+    ap.add_argument("-j", "--jobs", type=int, default=1)
+    args = ap.parse_args()
     util.build_oracle()
     fails = 0
-    for s in range(s0, s0 + n):
-        try:
-            desc, bad = one_case(s)
-        except Exception as e:   # a crash of either binary is a finding too
-            desc, bad = f"seed {s}", [f"EXCEPTION {str(e)[-300:]}"]
-        print(desc, "OK" if not bad else f"DIFF {bad}", flush=True)
-        fails += bool(bad)
+    with ThreadPoolExecutor(args.jobs) as ex:
+        for desc, bad in ex.map(checked, range(args.seed0, args.seed0 + args.n)):
+            print(desc, "OK" if not bad else f"DIFF {bad}", flush=True)
+            fails += bool(bad)
     sys.exit(1 if fails else 0)

@@ -65,6 +65,20 @@ CASES = [
 ]
 
 
+def _fuzz_cases():
+    """tests/test_oracle_fuzz.py, tests/test_gpu_fuzz.py: the run options synth.scenario_fuzz draws for each seed."""
+    out = []
+    with tempfile.TemporaryDirectory() as d:
+        for seed in util.FUZZ_SEEDS:
+            SCENARIOS[f"fuzz{seed}"] = (lambda s: lambda dd: synth.scenario_fuzz(dd, s)[0])(seed)
+            _cfg, K, flavour127, P, extra, _env = synth.scenario_fuzz(d, seed)
+            out.append((f"fuzz{seed}", flavour127, K, P, extra, False))
+    return out
+
+
+CASES += _fuzz_cases()
+
+
 def record(work, scenario, flavour127, K, P, extra, contig):
     ref = util.REF127 if flavour127 else util.REF63
     d = tempfile.mkdtemp(dir=work)

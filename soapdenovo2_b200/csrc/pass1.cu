@@ -85,7 +85,9 @@ void EngineT<NW>::chop_insert_chunk(const ReadChunk& ch) {
     const unsigned blocks = (unsigned)std::min<u64>((ch.n_rec + INS_THREADS - 1) / INS_THREADS, 148ull * 64);
     const size_t smem = (size_t)INS_THREADS * W64_ * sizeof(u64);
     const int use_tma = smem <= 96 * 1024;
-    if (use_tma && smem > 48 * 1024) cudaFuncSetAttribute(k_chop_insert<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    // opt in whatever the size: the kernel's static shared memory (barrier, counter) comes on top of the tile, so a 48 KB tile
+    // (max_rd_len 737..768) already exceeds the default limit
+    if (use_tma) PG_CUDA(cudaFuncSetAttribute(k_chop_insert<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k_chop_insert<NW><<<blocks, INS_THREADS, use_tma ? smem : 0, st_>>>(tab_, kp_, ch.words, ch.len, ch.n_rec, W64_, ch.ord_base, ch.ord_stride, d_cnt_, use_tma);
     pass_direct_ = true;
     if (inline_sweep_ == 1) inline_sweep_ = 2;   // entries swept by an aggregation launch have changed since

@@ -203,6 +203,10 @@ void EngineT<NW>::pass2(Pass2Stats* st, std::string* prearc_text, std::string* p
     std::vector<DevBuf> pathbufs(chunks_.size());
     DevBuf shared_path;
     if (!prm_.repsTie) shared_path.alloc(std::max<u64>(1, max_rec) * (u64)stride * sizeof(u32));
+    const size_t smem = (size_t)128 * W64_ * sizeof(u64);
+    const int use_tma = smem <= 48 * 1024 && !getenv("PGB200_NO_TMA");
+    // (the kernel's static shared memory comes on top of the tile: a 48 KB tile, max_rd_len 1505..1536, needs the opt-in)
+    if (use_tma) PG_CUDA(cudaFuncSetAttribute(k_pass2<NW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     for (size_t ci = 0; ci < chunks_.size(); ci++) {
         ReadChunk& c = chunks_[ci];
         if (!c.n_rec) continue;
@@ -210,8 +214,6 @@ void EngineT<NW>::pass2(Pass2Stats* st, std::string* prearc_text, std::string* p
         if (prm_.repsTie) { pathbufs[ci].alloc(c.n_rec * (u64)stride * sizeof(u32)); pb = pathbufs[ci].template as<u32>(); }
         else pb = shared_path.template as<u32>();
         unsigned blocks = (unsigned)std::min<u64>((c.n_rec + 127) / 128, 148ull * 32);
-        size_t smem = (size_t)128 * W64_ * sizeof(u64);
-        int use_tma = smem <= 48 * 1024 && !getenv("PGB200_NO_TMA");
         k_pass2<NW><<<blocks, 128, use_tma ? smem : 0, st_>>>(tab_, kp_, c.words, c.len, c.n_rec, W64_, c.ord_base, c.ord_stride, stride, pb,
                                              reclenb.template as<u32>(), prm_.repsTie, patch_buf_.template as<PatchSlot<NW>>(), patch_mask_,
                                              quirk128, arcs, acap - 1, markb.template as<u32>(), d_cnt_, errb.template as<u64>(), use_tma);

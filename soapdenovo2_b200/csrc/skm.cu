@@ -276,14 +276,15 @@ struct SmemTable {
 // One aggregated k-mer -> the global table.  A k-mer lives in exactly one bucket and a bucket is aggregated by one CTA at a time, so
 // when this call CLAIMS the slot nobody else can be touching its {payload, aux} words: they are written with one plain 16-byte store
 // (probe load -> claim CAS -> store: two dependent memory round trips per new key).  A key that already exists (earlier epoch: the
-// arena was flushed mid-stream) is merged with the same 64-bit CAS + atomicMin protocol every other writer uses.
-template <int NW>
-__device__ __forceinline__ bool table_merge(const Table<NW>& t, const Kmer<NW>& k, u64 agg, u64 rank) {
+// arena was flushed mid-stream; or instances of this bucket that were spilled) is merged with the same 64-bit CAS + atomicMin protocol
+// every other writer uses.  `on_claim` maps the aggregate to what a claimed slot stores; a merged aggregate is stored as it is.
+template <int NW, class OnClaim>
+__device__ __forceinline__ bool table_merge(const Table<NW>& t, const Kmer<NW>& k, u64 agg, u64 rank, OnClaim on_claim) {
     bool claimed;
     u64 idx = table_find_or_claim(t, k, &claimed);
     Slot<NW>* s = t.slots + idx;
     if (claimed) {
-        stcg128(&s->payload, U128{agg, rank});
+        stcg128(&s->payload, U128{on_claim(agg), rank});
         return true;
     }
     u64 cur = ldcg64(&s->payload);
@@ -554,18 +555,22 @@ __global__ void __launch_bounds__(SKM_APPLY_THREADS, SKM_APPLY_MIN_BLOCKS(NW)) k
             rb = rb_next;
         }
         __syncthreads();
-        // ---- flush: one global update per distinct k-mer of the bucket, walking the claim list (every thread busy)
+        // ---- flush: one global update per distinct k-mer of the bucket, walking the claim list (every thread busy).
+        // With a.sweep (this launch is the whole pass, into an empty table) an aggregate is swept only when this flush CLAIMS the key's
+        // global slot: every instance of the bucket has been applied (barrier above) and none of them reached the table, so the
+        // aggregate is the whole entry.  A key that is already there got there in this launch from instances of this bucket that
+        // were spilled (a warp saw its slot still empty and the claim count at the limit while another warp claimed it): that
+        // aggregate is partial, so it is merged unswept.  The first spilled instance put the slot on the spill list, which
+        // k_sweep_list sweeps after the launch, or found the list full, which makes the host sweep the whole table.
         const u32 n_claimed = s_count;
         for (u32 i = tid; i < n_claimed; i += SKM_APPLY_THREADS) {
             const u32 idx = st.list[i];
             Kmer<NW> k;
 #pragma unroll
             for (int w = 0; w < NW; w++) k.w[w] = st.key[w * SKM_SLOTS + idx];
-            u64 agg = st.pay[idx];
-            if (a.sweep) agg = sweep_payload(agg, a.D, sw_rem, sw_lin, s_hist);   // this launch is the whole pass: the entry is final
-            const bool fresh = table_merge(tab, k, agg, st.rnk[idx]);
+            const bool fresh = table_merge(tab, k, st.pay[idx], st.rnk[idx],
+                                           [&](u64 agg) { return a.sweep ? sweep_payload(agg, a.D, sw_rem, sw_lin, s_hist) : agg; });
             my_new += fresh;
-            if (a.sweep && !fresh) atomicAdd((unsigned long long*)&a.counters[C_SPILLKEYS], (unsigned long long)a.spill_cap + 1ull);   // (cannot happen in an empty table: makes the host run k_sweep)
             st.key[idx] = EMPTY64;
             st.pay[idx] = PAYLOAD_FRESH;
             st.rnk[idx] = ~0ull;
@@ -943,7 +948,9 @@ void EngineT<NW>::skm_flush_complete() {
     deferred[1] = deferred[0] + n_owned + 1;
     int launches = 1, which = 0;
     u64 n_def = h_flush_[3], maxu = h_flush_[4];
-    if (h_flush_[0]) throw std::runtime_error("pgb200: too many segments in one exchange epoch (flush more often)");
+    if (h_flush_[0])
+        throw std::runtime_error("pgb200: exchange arena overflow (the records of one chunk do not fit an arena half, or too many segments): "
+                                 "raise the arena capacity (pgb200_xchg_setup / PGB200_SKM_ARENA_MB) or feed smaller chunks");
     while (n_def) {
         // buckets whose worst case did not fit the table: grow so that (at least) the largest one fits, run them again
         read_counters();

@@ -204,6 +204,175 @@ def scenario_adversarial(d: str, seed=9, crlf=False, K_hint=31) -> str:
     return cfg
 
 
+# ---------------------------------------------------------------- seeded random scenarios (fuzzing the whole stage)
+FUZZ_K63 = (13, 15, 17, 21, 31, 33, 45, 61, 63)
+FUZZ_K127 = (63, 65, 67, 97, 99, 125, 127)
+# max_rd_len values at the edges of k_chop_insert's shared-memory modes (256 reads x ceil(L / 32) words: 48 KB / 96 KB)
+FUZZ_LONG_MAX = (768, 769, 1536, 1537)
+_IUPAC = b"RYKMSWBDHVrykmswbdhv"
+_DROPPED = b"0123456789-* \t"   # bytes the reader drops from a sequence line (not a letter, not '.')
+
+
+def _fuzz_seq(g, L, err, rng, junk):
+    """One read of L bases from g (either strand), substitution errors, then the scenario's unusual bytes (`junk`: subset of
+    'N', 'n', '.', 'lower', 'iupac', 'drop')."""
+    s = int(rng.integers(0, len(g) - L + 1))
+    r = g[s:s + L].copy()
+    if rng.random() < 0.5:
+        r = _COMP[r[::-1]]
+    if err > 0:
+        m = rng.random(L) < err
+        r[m] = _ACGT[(np.searchsorted(_ACGT, r[m]) + rng.integers(1, 4, size=int(m.sum()))) % 4]
+    return _fuzz_bytes(r, rng, junk)
+
+
+def _fuzz_bytes(r, rng, junk):
+    r = r.copy()
+    L = len(r)
+    if "lower" in junk and rng.random() < 0.2:
+        a, b = sorted(int(x) for x in rng.integers(0, L + 1, size=2))
+        r[a:b] |= 0x20
+    for c, sym in (("N", b"N"), ("n", b"n"), (".", b"."), ("iupac", _IUPAC)):
+        if c in junk and rng.random() < 0.08:
+            for _ in range(int(rng.integers(1, 4))):
+                r[int(rng.integers(0, L))] = sym[int(rng.integers(0, len(sym)))]
+    out = r.tobytes()
+    if "drop" in junk and rng.random() < 0.1:
+        for _ in range(int(rng.integers(1, 6))):
+            p = int(rng.integers(0, len(out) + 1))
+            out = out[:p] + bytes([_DROPPED[int(rng.integers(0, len(_DROPPED)))]]) * int(rng.integers(1, 3)) + out[p:]
+    return out
+
+
+def _write_fuzz_file(path, seqs, fastq, crlf, tag):
+    nl = b"\r\n" if crlf else b"\n"
+    with open(path, "wb") as f:
+        for i, s in enumerate(seqs):
+            if fastq:
+                f.write(b"@%s%d" % (tag, i) + nl + s + nl + b"+" + nl + b"I" * len(s) + nl)
+            else:
+                f.write(b">%s%d" % (tag, i) + nl + s + nl)
+    _pad_if_32k(path)
+
+
+def scenario_fuzz(d: str, seed: int):
+    """A random whole-stage scenario, deterministic from `seed`.  Returns (cfg, K, flavour127, P, extra, env): the config, the run
+    options (K, -p and the other flags of `pregraph`) and environment variables for the engine that select its insert path, chunk
+    size, table and bucket sizes, arena size, flush policy and TMA use (none of them may change the output).
+
+    Drawn independently: one to three libraries of f / q / f1+f2 / q1+q2 files (LF or CRLF per file), reverse_seq, rd_len_cutoff,
+    an asm_flags=2 library that must be ignored; ragged read lengths with exactly K+1 and multiples of 32 +-1; about one case in
+    six with 700-9000 bp reads and max_rd_len on either side of 768 and 1536 (lines longer than a 2 KB decode tile); max_rd_len
+    below the longest lines (truncation); N, n, '.', lower case, IUPAC letters and dropped bytes (digits, '-', '*', space, tab)
+    inside sequence lines; poly-A reads (saturated counters); K at the key-width and minimizer-length edges; -p, -a, -d, -R.
+
+    Shapes the reference itself mishandles are never drawn: '>' / '@' inside sequence lines, reads near 64 kbp, file sizes that are
+    multiples of 32 KiB, lines longer than its line buffers, and -R with long reads that could cross more than 255 edges (long-read
+    cases with -R are error-free)."""
+    rng = np.random.default_rng(seed)
+    flavour127 = int(rng.random() < 0.35)
+    K = int(rng.choice(FUZZ_K127 if flavour127 else FUZZ_K63))
+    P = int(rng.choice([1, 2, 3, 5, 8, 16]))
+    extra = []
+    a = int(rng.choice([0, 1, 2]))
+    if a:
+        extra += ["-a", str(a)]
+    D = int(rng.integers(0, 4))
+    if D:
+        extra += ["-d", str(D)]
+    rflag = bool(rng.random() < 0.5)
+    if rflag:
+        extra += ["-R"]
+    long_reads = bool(rng.random() < 1 / 6)
+    if long_reads:
+        max_rd_len = int(rng.choice(FUZZ_LONG_MAX)) if rng.random() < 0.6 else int(rng.integers(700, 9001))
+    else:
+        max_rd_len = max(K + 10, int(rng.choice([100, 128, 150, 160, int(rng.integers(K + 10, 200))])))
+    # The reference reads a line into a buffer of max(5000, max_rd_len + 1) bytes and carries a partial record over in one of
+    # 4 max_rd_len + 1024 bytes: longer lines overrun them.  16 bytes stay free for dropped bytes and a '\r'.
+    line_cap = max_rd_len if max_rd_len > 4900 else min(4900, 2 * max_rd_len + 400)
+    if long_reads:
+        top = int(rng.integers(max_rd_len, line_cap - 16 + 1)) if line_cap > max_rd_len else max_rd_len - 16   # longest read
+        glen = max(20000, 3 * top)
+    else:
+        top = max_rd_len + int(rng.choice([0, 0, 1, 20, 60]))               # > max_rd_len: truncation
+        glen = int(rng.integers(4000, 30000))
+    clean = long_reads and rflag   # error-free: a long read then crosses few edges
+    err = 0.0 if clean else float(rng.choice([0.0, 0.002, 0.006]))
+    junk = {c for c in ("N", "n", ".", "lower", "iupac", "drop") if rng.random() < 0.5}
+    if clean:
+        junk &= {"lower", "drop"}
+    g = genome(glen, seed, repeat=None if clean else (int(rng.integers(50, 400)), int(rng.integers(1, 4))))
+    lens_fixed = [K + 1, K + 1, 31, 32, 33, 63, 64, 65, 95, 96, 97, 127, 128, 129, max_rd_len - 1, max_rd_len, max_rd_len + 1, top]
+
+    def length():
+        if long_reads and rng.random() < 0.7:
+            L = int(rng.choice([max_rd_len, max_rd_len + 1, top])) if rng.random() < 0.3 else int(rng.integers(700, top + 1))
+        elif rng.random() < 0.4:
+            L = int(rng.choice(lens_fixed))
+        else:
+            L = int(rng.integers(max(K - 3, 13), min(top, 200) + 1))
+        return max(13, min(L, top, glen))
+
+    def seqs(n):
+        out = []
+        for _ in range(n):
+            if not clean and rng.random() < 0.03:
+                out.append(b"A" * int(rng.integers(K + 1, min(top, 200) + 1)))   # poly-A: links saturate at 63, coverage at 255
+            else:
+                out.append(_fuzz_seq(g, length(), err, rng, junk))
+        return out
+
+    budget = int(rng.integers(150_000, 600_000))   # bases per library
+    mean_len = (700 + top) / 2 * 0.7 + 100 * 0.3 if long_reads else min(top, 150)
+    libs = []
+    n_libs = int(rng.integers(1, 4))
+    ins = [int(x) for x in rng.choice(np.arange(150, 3000, 7), size=n_libs + 1, replace=False)]   # distinct: the sort order is defined
+    for li in range(n_libs):
+        kinds = [k for k in ("f", "q", "f12", "q12") if rng.random() < 0.45] or [str(rng.choice(["f", "q", "f12", "q12"]))]
+        files = []
+        per = max(40, int(budget / mean_len / len(kinds)))
+        for kind in kinds:
+            fq = kind.startswith("q")
+            tag = b"l%d%s" % (li, kind.encode())
+            if kind in ("f", "q"):
+                p = os.path.join(d, f"fz{li}_{kind}.{'fq' if fq else 'fa'}")
+                _write_fuzz_file(p, seqs(per), fq, bool(rng.random() < 0.3), tag)
+                files.append((kind, p))
+            else:
+                n = max(20, per // 2)
+                for m in (1, 2):
+                    p = os.path.join(d, f"fz{li}_{kind[0]}{m}.{'fq' if fq else 'fa'}")
+                    _write_fuzz_file(p, seqs(n), fq, bool(rng.random() < 0.3), tag)
+                    files.append((f"{kind[0]}{m}", p))
+        lib = {"avg_ins": ins[li], "reverse_seq": int(rng.random() < 0.25), "asm_flags": int(rng.choice([3, 3, 1])), "files": files}
+        if rng.random() < 0.25:
+            lib["rd_len_cutoff"] = int(rng.integers(K + 10, max_rd_len + 30))
+        libs.append(lib)
+    if rng.random() < 0.3:   # a library the pregraph stage must not read (asm_flags=2: scaffolding only)
+        p = os.path.join(d, "fz_ignored.fa")
+        _write_fuzz_file(p, seqs(50), False, False, b"ig")
+        libs.append({"avg_ins": ins[-1], "asm_flags": 2, "files": [("f", p)]})
+    cfg = os.path.join(d, "fuzz.cfg")
+    write_config(cfg, max_rd_len, libs)
+
+    env = {"PGB200_SKM": str(int(rng.integers(0, 2)))}
+    if rng.random() < 0.3:
+        env["PGB200_CHUNK_MB"] = "1"
+    if rng.random() < 0.25:
+        env["PGB200_TABLE_SLOTS"] = str(int(rng.choice([1024, 4096])))
+    if rng.random() < 0.3:
+        env["PGB200_SKM_BUCKETS"] = str(int(rng.choice([1, 3, 37, 256, 1024])))
+    if rng.random() < 0.2:   # a small arena (mid-stream aggregations) that still holds the records of one 1 MB chunk
+        env["PGB200_SKM_ARENA_MB"] = "64"
+        env["PGB200_CHUNK_MB"] = "1"
+    if rng.random() < 0.2:
+        env["PGB200_SKM_FLUSH_EVERY"] = str(int(rng.integers(1, 4)))
+    if rng.random() < 0.25:
+        env["PGB200_NO_TMA"] = "1"
+    return cfg, K, flavour127, P, tuple(extra), env
+
+
 # ---------------------------------------------------------------- vectorised writers for the config-sized cases (millions of reads)
 def _names(n: int, tag: bytes, width: int = 9) -> np.ndarray:
     ids = np.arange(n, dtype=np.int64)

@@ -106,6 +106,33 @@ def scenario_midsize(d):
     return cfg
 
 
+# Seeds of synth.scenario_fuzz with stored reference outputs (scenario names fuzz<seed>).  Chosen so that every edge the generator
+# aims at occurs: max_rd_len 768 (79), 769 (28 29 54 76), 1536 (5), 1537 (162) and above (53 92); lines longer than a 2 KB decode
+# tile (5 53 92); CRLF with truncation (1 5 10 ...); both insert paths, each with -d; PGB200_NO_TMA (10 14 23 ...); every K of both
+# builds, every -p, -a and -d; single-library cases (FUZZ_TABLE_SEEDS) whose pass-1 table is compared entry by entry.
+FUZZ_SEEDS = [1, 2, 5, 10, 14, 15, 20, 23, 24, 27, 28, 29, 32, 33, 36, 38, 44, 46, 48, 49, 50, 51, 52, 53, 54, 59, 60, 61, 63, 68,
+              70, 71, 72, 75, 76, 78, 79, 85, 86, 90, 92, 116, 149, 153, 156, 159, 162, 169]
+FUZZ_TABLE_SEEDS = [1, 2, 10, 23, 24, 27, 28, 32, 36, 38, 46, 49, 50, 53, 54, 59, 60, 63, 72, 78, 79, 85, 149, 156, 159, 169]
+
+
+def cfg_libs(cfg):
+    """Number of libraries of a config that the pregraph stage reads (asm_flags 1 or 3)."""
+    flags = [l.strip().split("=", 1)[1] for l in open(cfg) if l.startswith("asm_flags=")]
+    return sum(f in ("1", "3") for f in flags)
+
+
+def first_difference(a, b):
+    """'line N: <a line> != <b line>' for the first line where files a and b differ (.gz files are decompressed)."""
+    import gzip
+    op = gzip.open if a.endswith(".gz") else open
+    with op(a, "rb") as fa, op(b, "rb") as fb:
+        for n, (x, y) in enumerate(zip(fa, fb), 1):
+            if x != y:
+                return f"line {n}: {x[:200]!r} != {y[:200]!r}"
+        rest_a, rest_b = fa.read(), fb.read()
+    return f"one file is longer ({len(rest_a)} vs {len(rest_b)} trailing bytes)" if rest_a != rest_b else "no difference"
+
+
 def ref_key(scenario, flavour127, K, P, extra=()):
     return " ".join([scenario, "127mer" if flavour127 else "63mer", "-K", str(K), "-p", str(P), *extra])
 
